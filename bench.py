@@ -4,6 +4,7 @@
     python bench.py [--gpus N] [--steps K] [--warmup W]            # this repo's CUDA path (torchrun for N > 1)
     python bench.py --impl reference [--gpus N] [--steps K] ...    # the reference's CPU path on the host cores
     python bench.py --config {comb_1440,logoscan_10k,logo_analyze,logo_scan}   # secondary BASELINE configs, one JSON line
+    python bench.py --dump-outputs DIR ...                        # + the last timed step's results as DIR/{scores,counts}.npy
 
 One step = one pass of the fused hot path (LogoFrame::ScanFrame logo evaluation, 1 logo, fades {0,1}, + the
 combing / field-difference counters) over ONE synthetic 1800-frame 1920x1080i YV12 clip (BASELINE.json configs[1]),
@@ -125,6 +126,17 @@ class ClockSampler(threading.Thread):
                  "HwPowerBrakeSlowdown": "hw_power_brake_slowdown"}
         return {"sm_mhz": s[len(s) // 2], "sm_max_mhz": self.max_mhz, "reasons": sorted(snake[r] for r in self.reasons),
                 "samples": len(s)}
+
+
+def dump_outputs(d, scores, counts):
+    """--dump-outputs: what the timed path handed its caller in the last timed step, in one layout for every arm, one row per
+    clip (= per GPU): DIR/scores.npy float32 (clips, frames, 2) and DIR/counts.npy (clips, frames, 12), the int32 counters
+    widened to float64 (exact).  The inputs are seeded, so two builds run with the same arguments can be compared output
+    for output."""
+    import numpy as np
+    os.makedirs(d, exist_ok=True)
+    np.save(os.path.join(d, "scores.npy"), np.asarray(scores, np.float32).reshape(-1, CLIP_FRAMES, 2))
+    np.save(os.path.join(d, "counts.npy"), np.asarray(counts).astype(np.float64).reshape(-1, CLIP_FRAMES, 12))
 
 
 def make_clip(torch, synth, logo, device, seed, w=W, h=H, nframes=CLIP_FRAMES, mode="interlaced", imgx=IMGX, imgy=IMGY, out=None):
@@ -461,6 +473,8 @@ def run_group(args):
     launches = (c0.launches - l0) * n
     value = CLIP_FRAMES * n * args.steps / (elapsed_ms * 1e-3)
     d_scores, d_counts = g.fetch_results(CLIP_FRAMES, 0)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, d_scores, d_counts)
     # ---- end to end: pinned, NUMA-local host clips, one per GPU, staged concurrently by the members' own threads ----
     e2e = None
     hosts = []
@@ -541,7 +555,13 @@ def main():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-cpu", action="store_true", help="skip the CPU baseline AND the full-clip parity check")
     ap.add_argument("--no-secondary", action="store_true", help="skip the secondary configs in the headline line")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the results of the last timed step of the headline run (per-frame logo scores and combing "
+                         "counters) as DIR/scores.npy and DIR/counts.npy; not with --impl reference or --config")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl != "b200" or args.config != "headline"):
+        ap.error("--dump-outputs writes the results of the headline run of this repo's CUDA path: "
+                 "it cannot be combined with --impl reference or --config")
 
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -646,6 +666,12 @@ def main():
         comb_ms, comb_n = ctx.kernel_timing(reset=True)
         ctx.set_kernel_timing(False)
         launches = ctx.launches - l0
+    if args.dump_outputs and rank == 0:
+        if world > 1:                                     # every rank's results, as the last step's gather delivered them
+            r = gathered["results"]
+            dump_outputs(args.dump_outputs, r[:, : CLIP_FRAMES * 2].contiguous().view(torch.float32).cpu(), r[:, CLIP_FRAMES * 2:].cpu())
+        else:
+            dump_outputs(args.dump_outputs, scores.cpu(), counts.cpu())
     if world > 1:
         t = torch.tensor([elapsed_ms], dtype=torch.float64, device=device)
         dist.all_reduce(t, op=dist.ReduceOp.MAX)

@@ -416,10 +416,11 @@ def test_scan_logo_pipeline(ctx, oracle, tmp_path):
 def test_weave_frames_matches_mergefield(ctx):
     """AMTSource::MergeField/Copy1/Copy2 (AMTSource.hpp:291-355): even rows from `top`, odd rows from `bottom`,
     planar and NV12 sources, 8- and 16-bit."""
-    w, h, n = 208, 72, 6
-    src8 = synth.make_frames(0, n, w, h, device="cuda", mode="interlaced")
-    top = np.array([0, 1, 2, 3, 4, 5], np.int32)
-    bot = np.array([1, 2, 3, 4, 5, 5], np.int32)          # half-delay: bottom field of the next decoded frame
+    import ref_inputs as ri
+    w, h, n, top, bot = ri.WEAVE
+    src8 = ri.weave_frames("cuda")
+    top = np.array(top, np.int32)
+    bot = np.array(bot, np.int32)                         # half-delay: bottom field of the next decoded frame
     for bits in (8, 10):
         src = src8 if bits == 8 else (src8.to(torch.int32) * 4 + 2).to(torch.int16).contiguous()
         dst = torch.zeros_like(src)
@@ -447,10 +448,16 @@ def test_weave_frames_matches_mergefield(ctx):
     ref = torch.zeros_like(src8)
     ctx.weave_frames(ab.yv12_clip(src8, w, h, n, True), ab.yv12_clip(ref, w, h, n, True), top, bot)
     assert torch.equal(dst, ref)
-    # ... and both equal the reference's OWN MergeField / Copy1 / Copy2 (compiled from AMTSource.hpp:291-355 into oracle/_ref)
+    # ... and both equal the reference's OWN MergeField / Copy1 / Copy2 (AMTSource.hpp:291-355; its outputs stored as digests
+    # in tests/golden/ref_cases.json, and computed live where oracle/_ref is built)
+    import hashlib
     from oracle import pyoracle as po
+    gw = json.load(open(os.path.join(os.path.dirname(__file__), "golden", "ref_cases.json")))["weave"]
+    g = dst.cpu().numpy()
+    for k in range(n):
+        sha = hashlib.sha256(np.ascontiguousarray(g[k]).tobytes()).hexdigest()
+        assert sha == gw["planar_sha"][k] and sha == gw["nv12_sha"][k], k
     if po.ref_has_mergefield():
-        g = dst.cpu().numpy()
         for k in range(n):
             assert np.array_equal(g[k], po.ref_merge_field(a[top[k]], a[bot[k]], w, h)), ("planar", k)
             assert np.array_equal(g[k], po.ref_merge_field(nv[top[k]], nv[bot[k]], w, h, nv12=True)), ("nv12", k)

@@ -3,26 +3,34 @@ tiles, a quarter-used last tile column, 5.625 chroma tiles), 8- and 10-bit, agai
 (LogoScan accumulation over 10000 1920x1080 frames, ROI 64x64 and 256x128) against the reference's own LogoScan code
 (oracle/_ref) where it exists, else the C port; a whole 1080p clip against the reference-compiled logo code.  Everything
 goes through the C ABI."""
+import hashlib
+import json
+import os
+
 import numpy as np
 import pytest
 import torch
 
 import amatsukaze_b200 as ab
+import ref_inputs as ri
 from amatsukaze_b200 import synth
 
 pytestmark = pytest.mark.gpu
+# the reference's own results at these sizes (tests/golden/gen_golden.py --sizes): the comparison with the reference holds
+# where oracle/_ref is not built
+REF = json.load(open(os.path.join(os.path.dirname(__file__), "golden", "ref_sizes.json")))
 
 
 def _bits(a):
     return np.ascontiguousarray(a, np.float32).view(np.uint32)
 
 
+def _digest(a):
+    return hashlib.sha256(np.ascontiguousarray(a).tobytes()).hexdigest()
+
+
 def _gen(n0, n, w, h, **kw):
-    out = torch.empty((n, w * h * 3 // 2), dtype=torch.uint8, device="cuda")
-    for k in range(0, n, 10):
-        m = min(10, n - k)
-        synth.make_frames(n0 + k, m, w, h, device="cuda", out=out[k:k + m], **kw)
-    return out
+    return ri.gen_frames(n0, n, w, h, "cuda", **kw)
 
 
 @pytest.mark.timeout(900)
@@ -63,9 +71,9 @@ def test_comb_1440x1080_8bit_and_10bit(ctx, oracle):
 def test_scan_and_analyze_1440x1080(ctx, oracle):
     """configs[0]'s geometry (1440x1080, 64x64 template at (1280, 64)) on the GPU, against the reference's own code."""
     po = oracle
-    w, h, n, imgx, imgy = 1440, 1080, 16, 1280, 64
+    w, h, n, imgx, imgy = ri.SCAN_1440
     lg = synth.make_logo(64, 64)
-    fr = _gen(35, n, w, h, logo=lg, imgx=imgx, imgy=imgy, logo_period=16)
+    fr = ri.scan_1440_frames(lg, "cuda")
     raw = ab.Logo.create(lg["data"], 64, 64, w, h, imgx, imgy)
     de, top, bot = raw.deint().create_mask(0.35), raw.field(0).create_mask(0.35), raw.field(1).create_mask(0.35)
     clip = ab.yv12_clip(fr, w, h, n, True)
@@ -85,6 +93,9 @@ def test_scan_and_analyze_1440x1080(ctx, oracle):
     assert np.array_equal(_bits(s[:, 0]), _bits(rs))
     assert np.array_equal(_bits(a[0:n:5]), _bits(ra))
     assert rs[:, 0].max() > 0.5 and rs[:, 0].min() < 0.2
+    g = REF["scan_analyze_1440"]
+    assert _bits(s[:, 0]).ravel().tolist() == g["scan_bits"]
+    assert g["analyze_frames"] == list(range(0, n, 5)) and _bits(a[0:n:5]).ravel().tolist() == g["analyze_bits"]
 
 
 @pytest.mark.timeout(1800)
@@ -92,17 +103,17 @@ def test_logoscan_10000_frames_1080p(ctx, oracle):
     """configs[3]: 10000 resident 1920x1080 frames (31 GB), ROI 64x64 and 256x128: u64 sums, gridDim.y frame splits,
     validity per frame, and the derived logo (A/B planes) -- all exact."""
     po = oracle
-    w, h, n = 1920, 1080, 10000
+    w, h, n = ri.LOGOSCAN_10K
     free, _ = torch.cuda.mem_get_info()
     if free < 36 * (1 << 30):
         pytest.skip("needs 36 GB of free HBM")
     lg = synth.make_logo(64, 64)
     fr = torch.empty((n, w * h * 3 // 2), dtype=torch.uint8, device="cuda")
     for k in range(0, n, 20):
-        synth.make_frames(k, 20, w, h, seed=0x5EED0007, device="cuda", mode="flat", logo=lg, imgx=1700, imgy=60, out=fr[k:k + 20])
+        ri.logoscan_10k_frames(k, 20, lg, "cuda", out=fr[k:k + 20])
     clip = ab.yv12_clip(fr, w, h, n, True)
     ysz, csz = w * h, (w // 2) * (h // 2)
-    for (sx, sy, sw, sh) in ((1700, 60, 64, 64), (1600, 60, 256, 128)):
+    for (sx, sy, sw, sh) in ri.LOGOSCAN_10K_ROIS:
         acc = ctx.logo_scan(sw, sh, 12)
         valid = acc.add_frames(clip, sx, sy, 0, 6000)
         valid = np.concatenate([valid, acc.add_frames(clip, sx, sy, 6000, 4000)])        # accumulates across calls
@@ -115,9 +126,13 @@ def test_logoscan_10000_frames_1080p(ctx, oracle):
         assert np.array_equal(valid, ov), (sw, sh, int((valid != ov).sum()))
         assert 0 < int(ov.sum()) < n and acc.num_valid == o.nframes == int(ov.sum())
         assert np.array_equal(acc.sums(), o.sums())              # exact integers (< 2^53) in doubles
+        g = REF["logoscan_10k"]["%dx%d" % (sw, sh)]
+        assert _digest(valid.astype(np.uint8)) == g["valid_sha"] and acc.num_valid == g["nframes"]
+        assert _digest(acc.sums()) == g["sums_sha"]
         for clean in (False, True):
             a, b = acc.get_logo(255, clean), o.get_logo(255, clean)
             assert a is not None and b is not None and np.array_equal(a.view(np.uint32), b.view(np.uint32))
+            assert _digest(a) == g["logo_clean_sha" if clean else "logo_sha"]
         del acc
 
 
@@ -127,9 +142,9 @@ def test_whole_clip_1080p_against_reference_code(ctx, oracle):
     32-, 8- and 4-frame items): every logo score bit-identical with the reference's own compiled code, every combing
     counter identical with the spec (AVX2 form; scalar form on a subset)."""
     po = oracle
-    w, h, n, imgx, imgy = 1920, 1080, 1000, 1700, 60
+    w, h, n, imgx, imgy = ri.WHOLE_CLIP
     lg = synth.make_logo(64, 64)
-    fr = _gen(0, n, w, h, logo=lg, imgx=imgx, imgy=imgy)
+    fr = ri.whole_clip_frames(lg, "cuda")
     logo = ab.Logo.create(lg["data"], 64, 64, w, h, imgx, imgy).deint().create_mask(0.35)
     prm = ab.default_comb_params()
     s, c = ctx.scan_comb_frames(ab.yv12_clip(fr, w, h, n, True), [logo], prm)
@@ -140,6 +155,7 @@ def test_whole_clip_1080p_against_reference_code(ctx, oracle):
     _, _, rc_s = b.run(host[:24], prm.as_list(), 2, "scalar")
     b.close()
     assert np.array_equal(_bits(s[:, 0]), _bits(rs))
+    assert _digest(_bits(s[:, 0])) == REF["whole_clip_1080p"]["scores_sha"] and REF["whole_clip_1080p"]["frames"] == n
     assert np.array_equal(c, rc) and np.array_equal(c[:24], rc_s)
     # host-buffer path over the same clip (staged through HBM by the library): identical
     s2, c2 = ctx.scan_comb_frames(ab.yv12_clip(host, w, h, n, False), [logo], prm)

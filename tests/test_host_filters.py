@@ -1,6 +1,7 @@
 """The host-side C++ mirror of the reference's filter interface (amatsukaze_b200/host/filters.hpp), driven by
 tests/cpp/test_filters.cpp the way CMAnalyze::logoFrame and AMTFilterSource drive the reference, checked against the
-oracle (and against the reference's own LogoFrame::selectLogo/writeResult where oracle/_ref is present)."""
+oracle and against the reference's own LogoFrame::selectLogo/writeResult (stored results; live where oracle/_ref is built)."""
+import json
 import os
 import struct
 import subprocess
@@ -9,11 +10,13 @@ import numpy as np
 import pytest
 
 import amatsukaze_b200 as ab
+import ref_inputs as ri
 from amatsukaze_b200 import synth, _build
 from oracle import pyoracle as po
 
 pytestmark = pytest.mark.gpu
-W, H, N, IMGX, IMGY = 256, 128, 61, 160, 32
+W, H, N, IMGX, IMGY = ri.FILTERS_CLIP
+REF = json.load(open(os.path.join(os.path.dirname(__file__), "golden", "ref_cases.json")))
 
 
 def _bits(a):
@@ -24,8 +27,7 @@ def _bits(a):
 def run(tmp_path_factory):
     exe = _build.build_host_test() if os.path.exists("/usr/bin/g++") else _build.HOST_TEST
     out = tmp_path_factory.mktemp("filters")
-    lg = synth.make_logo(64, 64, seed=1)
-    frames = synth.make_frames(35, N, W, H, logo=lg, imgx=IMGX, imgy=IMGY, logo_period=40).numpy()
+    lg, frames = ri.filters_clip()
     clip = out / "clip.amtsraw"
     with open(clip, "wb") as f:
         f.write(b"AMTSRAW1" + struct.pack("<6i", W, H, 8, N, 30000, 1001))
@@ -56,11 +58,14 @@ def test_logoframe_scan_select_write(run):
     assert np.all(ev[:, 1, 0] == 0) and np.all(ev[:, 1, 1] == -1)            # unreadable logo file -> (0,-1)
     txt = open(out / "logof.txt").read()
     assert "bestLogo=0" in run["stdout"]
+    # the reference's selectLogo / writeResult on these scores (tests/golden/ref_cases.json; live where oracle/_ref is built)
+    g = REF["filters_logoframe"]["fps"]["30"]
+    best, ratio = g["best"], float(np.uint32(g["ratio_bits"]).view(np.float32))
+    assert best == 0 and ("logoRatio=%.6f" % ratio) in run["stdout"]
+    assert txt == g["text"] and len(txt.splitlines()) >= 2
     if po.ref_available():
         rp = str(out / "logof_ref.txt")
-        best, ratio = po.ref_logoframe(ev, 30, rp)
-        assert best == 0 and ("logoRatio=%.6f" % ratio) in run["stdout"]
-        assert txt == open(rp).read() and len(txt.splitlines()) >= 2
+        assert po.ref_logoframe(ev, 30, rp) == (best, ratio) and open(rp).read() == txt
 
 
 def test_cmanalyze_logoframe_entry(run):
@@ -75,16 +80,24 @@ def test_cmanalyze_logoframe_entry(run):
 
 
 def test_logoframe_write_result_matches_reference_on_many_patterns(run, tmp_path):
-    """selectLogo/writeResult are pure host code: exercise them on synthetic score tracks against the reference's own
-    implementation (oracle/_ref, LogoScan.hpp:1645-1827 compiled verbatim)."""
-    if not po.ref_available():
-        pytest.skip("oracle/_ref not built")
-    # the C++ class is exercised through the test driver only for the clip above; here the reference implementation
-    # pins the expected file for that clip's scores under different frame rates
+    """selectLogo/writeResult are pure host code: the product's (tests/cpp/test_host_only.cpp driver) on the clip's scores
+    under different frame rates against the reference's own implementation (LogoScan.hpp:1645-1827; results stored in
+    tests/golden/ref_cases.json, and oracle/_ref live where it is built)."""
     ev = np.fromfile(run["out"] / "eval.bin", np.float32).reshape(N, 2, 2)
-    for fps in (24, 30, 60):
-        best, ratio = po.ref_logoframe(ev, fps, str(tmp_path / ("r%d.txt" % fps)))
+    exe = _build.build_host_only_test()
+    for fps in ri.FILTERS_LOGOFRAME_FPS:
+        g = REF["filters_logoframe"]["fps"][str(fps)]
+        best, ratio = g["best"], np.uint32(g["ratio_bits"]).view(np.float32)
         assert best == 0 and 0.0 < ratio < 1.0
+        if po.ref_available():
+            assert po.ref_logoframe(ev, fps, str(tmp_path / ("r%d.txt" % fps))) == (best, float(ratio))
+            assert open(tmp_path / ("r%d.txt" % fps)).read() == g["text"]
+        sp, op = tmp_path / "s.bin", tmp_path / ("o%d.txt" % fps)
+        ev.tofile(sp)
+        r = subprocess.run([exe, "logoframe", str(sp), str(N), "2", str(fps), "1", str(op)], capture_output=True, text=True, timeout=120)
+        assert r.returncode == 0, r.stdout + r.stderr
+        assert ("bestLogo=%d " % best) in r.stdout and np.float32(float(r.stdout.split("logoRatio=")[1])) == ratio, (fps, r.stdout)
+        assert open(op).read() == g["text"], fps
 
 
 def test_analyze_records_and_fades(run):

@@ -1,7 +1,9 @@
 """Host-side logic of the filter mirror that needs no device (tests/cpp/test_host_only.cpp): LogoFrame::selectLogo /
-writeResult against the reference's own code (oracle/_ref, LogoScan.hpp:1645-1827 compiled verbatim), AMTEraseLogo's
+writeResult against the reference's own code (LogoScan.hpp:1645-1827; results stored in tests/golden/ref_cases.json, and
+oracle/_ref live where it is built), AMTEraseLogo's
 logoframe state machine + fade selection against the oracle's CalcFade2, AMTDecimate, the timecode reader and the
 telecine side files.  CPU suite."""
+import json
 import os
 import subprocess
 
@@ -9,8 +11,11 @@ import numpy as np
 import pytest
 
 import amatsukaze_b200 as ab
+import ref_inputs as ri
 from amatsukaze_b200 import _build, synth
 from oracle import pyoracle as po
+
+REF = json.load(open(os.path.join(os.path.dirname(__file__), "golden", "ref_cases.json")))
 
 
 @pytest.fixture(scope="module")
@@ -24,43 +29,25 @@ def run(exe, *args, ok=(0,)):
     return r
 
 
-def score_track(rng, n, on_ranges, noise=0.08, flicker=0.0):
-    """(n, 2) corr0/corr1 as ScanFrame produces them: logo present -> corr0 high, corr1 ~ 0; absent -> corr0 ~ 0, corr1 < 0."""
-    on = np.zeros(n, bool)
-    for a, b in on_ranges:
-        on[a:b] = True
-    if flicker:
-        on ^= rng.random(n) < flicker
-    c0 = np.where(on, 0.8, 0.0) + rng.normal(0, noise, n)
-    c1 = np.where(on, 0.0, -0.8) + rng.normal(0, noise, n)
-    return np.stack([c0, c1], 1).astype(np.float32)
-
-
-@pytest.mark.parametrize("fps", [(24000, 1001), (30000, 1001), (60000, 1001), (25, 1)])
+@pytest.mark.parametrize("fps", ri.LOGOFRAME_FPS)
 def test_logoframe_select_and_write_match_reference(exe, tmp_path, fps):
-    if not po.ref_available():
-        pytest.skip("oracle/_ref not built")
-    rng = np.random.default_rng(fps[0])
+    """The product's LogoFrame::selectLogo / writeResult against the reference's results on the same score tracks (stored in
+    tests/golden/ref_cases.json; also computed live where oracle/_ref is built)."""
     n = 700
-    cases = [
-        [[(100, 400)], [(0, 0)]],                                   # one section, second logo never present
-        [[(0, 250), (400, 700)], [(50, 120)]],                      # starts and ends inside a section
-        [[(60, 90), (130, 170), (300, 650)], [(0, 700)]],           # short sections, always-on competitor
-        [[(0, 0)], [(0, 0)]],                                       # nothing anywhere
-        [[(0, 700)], [(200, 500)]],                                 # everything
-        [[(200, 210), (215, 500)], [(10, 20)]],                     # a gap shorter than the filters
-    ]
-    for ci, (a, b) in enumerate(cases):
-        for flicker in (0.0, 0.03):
-            ev = np.stack([score_track(rng, n, a, flicker=flicker), score_track(rng, n, b, flicker=flicker)], 1)   # (n, 2 logos, 2)
+    want = iter(REF["logoframe"]["%d/%d" % fps])
+    for ci, flicker, ev in ri.logoframe_tracks(fps):              # ev: (n, 2 logos, 2)
             sp, op, rp = tmp_path / "s.bin", tmp_path / "o.txt", tmp_path / "r.txt"
             ev.tofile(sp)
             r = run(exe, "logoframe", sp, n, 2, fps[0], fps[1], op)
-            best, ratio = po.ref_logoframe(ev, int(round(fps[0] / fps[1])), str(rp))
+            g = next(want)
+            best, ratio, text = g["best"], np.uint32(g["ratio_bits"]).view(np.float32), g["text"]
+            if po.ref_available():
+                live = po.ref_logoframe(ev, int(round(fps[0] / fps[1])), str(rp))
+                assert live == (best, float(ratio)) and open(rp).read() == text, (ci, flicker)
             assert ("bestLogo=%d " % best) in r.stdout, (ci, flicker, r.stdout, best)
             got_ratio = float(r.stdout.split("logoRatio=")[1])
-            assert np.float32(got_ratio) == np.float32(ratio)
-            assert open(op).read() == open(rp).read(), (ci, flicker)
+            assert np.float32(got_ratio) == ratio
+            assert open(op).read() == text, (ci, flicker)
 
 
 def test_timecode_reader(exe, tmp_path):
@@ -101,40 +88,39 @@ def test_decimate_map_and_mismatch(exe, tmp_path):
 
 def test_sidefile_readers_equal_the_reference_code(exe, tmp_path):
     """The product's TimecodeFile and AMTDecimate (host/filters.hpp) against the reference's OWN readTimecodeFile + base-fps
-    estimate and AMTDecimate constructor/GetFrame, compiled from FilteredSource.hpp:163-188,197-210,645-660,663-666 into
-    oracle/_ref: same time codes (compared at the driver's printed 1e-6 ms resolution), same vfrTimingFps, same frame map, same
-    mismatch message; edge cases: empty file, one stamp, total line with trailing text, CRLF, comments, no total line."""
-    if not (po.ref_available() and po.ref_has_sidefiles()):
-        pytest.skip("oracle/_ref (with the side-file readers) not built: needs /root/reference")
-    rng = np.random.default_rng(3)
-    cases = []
-    for grid in (60, 120, 240, 0):
-        t, stamps = 0.0, []
-        for _ in range(int(rng.integers(2, 90))):
-            stamps.append(int(round(t)))
-            t += (1001.0 / grid * 1000.0 / 1000.0 * int(rng.integers(1, 4)) * (1000.0 / 1000.0)) if grid else float(rng.integers(5, 80))
-        body = "# timecode format v2\n" + "".join("%d\n" % v for v in stamps)
-        cases += [body + "# total: %.3f\n" % (t / 1000.0), body, body + "\r\n#comment\n\n"]
-    cases += ["", "17\n", "# total: 12.5\n", "5\n9\n# total: 1.0 trailing\n33\n"]
+    estimate and AMTDecimate constructor/GetFrame (FilteredSource.hpp:163-188,197-210,645-660,663-666; their results on these
+    files are stored in tests/golden/ref_cases.json and also computed live where oracle/_ref is built): same time codes
+    (compared at the driver's printed 1e-6 ms resolution), same vfrTimingFps, same frame map, same mismatch message; edge
+    cases: empty file, one stamp, total line with trailing text, CRLF, comments, no total line."""
+    live = po.ref_has_sidefiles()
+    g = REF["sidefiles"]
+    cases, durations = ri.sidefile_inputs()
+    assert len(cases) == len(g["timecode"])
     for k, text in enumerate(cases):
         p = tmp_path / ("tc%d.txt" % k)
         p.write_bytes(text.encode())
         out = run(exe, "timecode", p).stdout.split()
-        codes, fps = po.ref_read_timecode(p)
+        codes, fps = g["timecode"][k]["codes"], g["timecode"][k]["fps"]
+        if live:
+            assert po.ref_read_timecode(p) == (codes, fps), k
         assert out[0] == "ok=1" and out[1] == "n=%d" % len(codes) and out[2] == "fps=%d" % fps, (k, out[:3], len(codes), fps)
         assert [float(x) for x in out[3:]] == [float("%.6f" % c) for c in codes], k
-    assert po.ref_read_timecode(tmp_path / "missing.txt") is None and "ok=0" in run(exe, "timecode", tmp_path / "missing.txt").stdout
-    for k in range(8):
-        dur = [int(v) for v in rng.integers(1, 4, size=int(rng.integers(1, 60)))]
+    assert "ok=0" in run(exe, "timecode", tmp_path / "missing.txt").stdout
+    if live:
+        assert po.ref_read_timecode(tmp_path / "missing.txt") is None
+    for k, dur in enumerate(durations):
         d = tmp_path / ("dur%d.txt" % k)
         d.write_text("".join("%d\n" % v for v in dur))
-        want = po.ref_decimate_map(d, sum(dur))
+        want, err = g["decimate"][k]["map"], g["decimate"][k]["mismatch_error"]
+        if live:
+            assert po.ref_decimate_map(d, sum(dur)) == want
+            with pytest.raises(RuntimeError) as ei:
+                po.ref_decimate_map(d, sum(dur) + 1)
+            assert str(ei.value).replace(str(d), "<path>") == err
         out = run(exe, "decimate", d, sum(dur)).stdout
         assert out.split("map:")[0].strip() == "frames=%d" % len(want) and [int(x) for x in out.split("map:")[1].split()] == want
-        with pytest.raises(RuntimeError) as ei:
-            po.ref_decimate_map(d, sum(dur) + 1)
         r = run(exe, "decimate", d, sum(dur) + 1, ok=(4,))
-        assert "[AMTDecimate] # of frames does not match." in str(ei.value) and str(ei.value).split("]")[1].strip().split("(")[0] in r.stdout
+        assert "[AMTDecimate] # of frames does not match." in err and err.split("]")[1].strip().split("(")[0] in r.stdout
 
 
 def test_telecine_side_files_from_counts(exe, tmp_path):
@@ -182,9 +168,7 @@ def _frame_result(n, elems):
 
 
 def test_eraselogo_fade_selection(exe, tmp_path):
-    n, maxfade = 120, 16
-    rng = np.random.default_rng(11)
-    rec = rng.normal(0.0, 0.5, (n, 33)).astype(np.float32)
+    n, maxfade, rec, elems = ri.erase_fades_inputs()
     rp = tmp_path / "rec.bin"
     rec.tofile(rp)
     lg = synth.make_logo(32, 32, seed=2)
@@ -197,9 +181,8 @@ def test_eraselogo_fade_selection(exe, tmp_path):
     want = np.array([po.or_calc_fade2(rec, n, i) for i in range(n)], np.float32)
     assert np.array_equal(got.view(np.uint32), want.view(np.uint32))
     # with one: frames whose +-maxfade/2 neighbourhood has a uniform state take 0 / 1 directly (:1317-1341)
-    elems = [((22, 20, 26), (58, 55, 61)), ((90, 88, 93), (118, 115, 119))]
     lf = tmp_path / "logof.txt"
-    lf.write_text("".join("%6d S 0 ALL %6d %6d\n%6d E 0 ALL %6d %6d\n" % (*s, *e) for s, e in elems))
+    lf.write_text(ri.logoframe_file(elems))
     run(exe, "fades", lp, lf, rp, n, maxfade, fp)
     got = np.fromfile(fp, np.float32).reshape(n, 2)
     fr = _frame_result(n, elems)
@@ -215,7 +198,13 @@ def test_eraselogo_fade_selection(exe, tmp_path):
         assert tuple(np.float32(exp)) == tuple(got[i]), i
     assert 0 < direct < n
     # ... and so does the reference's OWN ReadLogoFrameFile + CalcFade (LogoScan.hpp:1317-1341,1421-1461; compiled from the
-    # reference's lines into oracle/_ref): the product's C++ driver picks the same fades, frame for frame, bit for bit
+    # reference's lines into oracle/_ref, its results stored in tests/golden/ref_cases.json): the product's C++ driver picks
+    # the same fades, frame for frame, bit for bit
+    g = REF["erase_fades"]
+    assert np.array_equal(np.array(g["state"], np.int32), fr)
+    assert got.view(np.uint32).ravel().tolist() == g["logof_bits"]
+    assert want.view(np.uint32).ravel().tolist() == g["no_logof_bits"]
+    assert "Start and End must be cyclic" in g["cyclic_error"]
     if po.ref_available() and hasattr(po.ref_lib(), "ref_erase_fades"):
         rf, rstate = po.ref_erase_fades(rec, n, lf, maxfade)
         assert np.array_equal(rstate, fr)

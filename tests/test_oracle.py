@@ -1,6 +1,7 @@
 """CPU tests of the checker itself: the plain-C oracle (oracle/amtk_oracle.c) must reproduce
   (1) the committed golden vectors the REFERENCE'S OWN code produced (tests/golden/logo_golden.json), always;
-  (2) the reference's own compiled code (oracle/_ref) live, when that library is present.
+  (2) the reference's results on further cases, stored in tests/golden/ref_cases.json, and the reference's own compiled
+      code (oracle/_ref) live, when that library is present.
 All float comparisons are on bit patterns."""
 import ctypes as C
 import hashlib
@@ -10,12 +11,13 @@ import os
 import numpy as np
 import pytest
 
+import ref_inputs as ri
 from amatsukaze_b200 import synth
 from oracle import pyoracle as po
 
 GOLD = json.load(open(os.path.join(os.path.dirname(__file__), "golden", "logo_golden.json")))
+REF = json.load(open(os.path.join(os.path.dirname(__file__), "golden", "ref_cases.json")))
 W, H, IMGX, IMGY = 256, 128, 160, 32
-needs_ref = pytest.mark.skipif(not po.ref_available(), reason="oracle/_ref not built (needs /root/reference)")
 
 
 def bits(a):
@@ -107,139 +109,140 @@ def test_logoscan_insufficient_frames_returns_none():
     assert sc.get_logo(255) is None      # 0 frames -> NaN slopes -> the reference returns nullptr (LogoScan.hpp:391,503)
 
 
-@needs_ref
+def _port_logo_tables(o, planes, maxv):
+    return {"count": o.s.count, "maskpixels": o.s.maskpixels, "mask_sha": digest(o.mask()), "kernels_sha": digest(o.kernels()),
+            "scales_sha": digest(o.scales()), "black_bits": bits([o.s.blackScore])[0],
+            "scan_bits": [bits(o.scan_frame(p, maxv=maxv)) for p in planes]}
+
+
 def test_oracle_equals_reference_live():
     """Random logos / frames beyond the golden set, incl. 16-bit samples, odd sizes and a logo whose mask
-    spills into zero-variance pixels (count < maskpixels, SURVEY 8 quirks)."""
-    rng = np.random.default_rng(7)
-    for case, (w, h, ratio, bitsps) in enumerate(((64, 64, 0.35, 8), (48, 40, 0.9, 8), (64, 32, 0.35, 10), (32, 64, 0.1, 8))):
-        lg = synth.make_logo(w, h, seed=case)
-        data = lg["data"].copy()
-        if case == 1:
-            data[: w * h][(rng.random(w * h) < 0.3)] *= 1.0      # keep flat areas: high maskratio forces border picks
-        fw, fh, ix, iy = 320, 200, 100, 60
-        r = po.RefLogo.create(data, w, h, fw, fh, ix, iy).deint().create_mask(ratio)
+    spills into zero-variance pixels (count < maskpixels, SURVEY 8 quirks).  The reference's results are stored in
+    tests/golden/ref_cases.json; where oracle/_ref is built, the reference is also run live."""
+    fw, fh, ix, iy = ri.LOGO_FRAME
+    for case, w, h, data, ratio, maxv, planes in ri.logo_cases():
         o = po.OracleLogo.create(data, w, h, fw, fh, ix, iy).deint().create_mask(ratio)
-        assert r.visited_count() == o.s.count and r.dims()["maskpixels"] == o.s.maskpixels
-        assert np.array_equal(r.mask(), o.mask())
-        assert np.array_equal(r.kernels().view(np.uint32), o.kernels().view(np.uint32))
-        assert np.array_equal(r.scales().view(np.uint32), o.scales().view(np.uint32))
-        assert bits([r.black_score()]) == bits([o.s.blackScore])
-        maxv = float((1 << bitsps) - 1)
-        for _ in range(4):
-            if bitsps == 8:
-                plane = rng.integers(16, 236, (fh, fw), dtype=np.uint8)
-            else:
-                plane = rng.integers(64, 940, (fh, fw)).astype(np.uint16)
-            assert bits(po.ref_scan_frame(r, plane, maxv)) == bits(o.scan_frame(plane, maxv=maxv))
+        got = _port_logo_tables(o, planes, maxv)
+        assert got == REF["logos"][case], case
+        if po.ref_available():
+            r = po.RefLogo.create(data, w, h, fw, fh, ix, iy).deint().create_mask(ratio)
+            assert np.array_equal(r.mask(), o.mask()) and r.visited_count() == o.s.count
+            assert np.array_equal(r.kernels().view(np.uint32), o.kernels().view(np.uint32))
+            assert np.array_equal(r.scales().view(np.uint32), o.scales().view(np.uint32))
+            assert [bits(po.ref_scan_frame(r, p, maxv)) for p in planes] == got["scan_bits"]
         if case == 1:
             assert o.s.count < o.s.maskpixels          # the quirk case really happened
 
 
-@needs_ref
 def test_oracle_logoscan_equals_reference_live():
-    rng = np.random.default_rng(11)
-    ro, oo = po.RefScan(24, 16, 10), po.OracleScan(24, 16, 10)
-    for i in range(60):
-        base = int(rng.integers(30, 200))
-        y = (base + rng.integers(-3, 4, (16, 24))).astype(np.uint8)
-        if i % 7 == 0:
-            y[0, 3] = 255                               # breaks the flat-border test
-        u = (128 + rng.integers(-2, 3, (8, 12))).astype(np.uint8)
-        v = (128 + rng.integers(-2, 3, (8, 12))).astype(np.uint8)
-        y[4:12, 6:18] = np.clip(y[4:12, 6:18].astype(int) + 40, 0, 255).astype(np.uint8)
-        assert ro.add_frame(y, u, v) == oo.add_frame(y, u, v)
-    assert ro.nframes == oo.nframes
-    assert np.array_equal(ro.sums(), oo.sums())
-    for clean in (False, True):
-        a, b = ro.get_logo(255, clean), oo.get_logo(255, clean)
-        assert (a is None) == (b is None)
-        if a is not None:
-            assert np.array_equal(a.view(np.uint32), b.view(np.uint32))
+    ro = po.RefScan(24, 16, 10) if po.ref_available() else None
+    oo = po.OracleScan(24, 16, 10)
+    g = REF["logoscan"]
+    for i, (y, u, v) in enumerate(ri.logoscan_frames()):
+        assert oo.add_frame(y, u, v) == g["valid"][i]
+        if ro is not None:
+            assert ro.add_frame(y, u, v) == g["valid"][i]
+    assert oo.nframes == g["nframes"]
+    assert digest(oo.sums()) == g["sums_sha"]
+    for k, clean in enumerate((False, True)):
+        b = oo.get_logo(255, clean)
+        assert (None if b is None else digest(b)) == g["logo_sha"][k]
+    if ro is not None:
+        assert ro.nframes == oo.nframes and np.array_equal(ro.sums(), oo.sums())
+        for clean in (False, True):
+            a, b = ro.get_logo(255, clean), oo.get_logo(255, clean)
+            assert (a is None) == (b is None)
+            if a is not None:
+                assert np.array_equal(a.view(np.uint32), b.view(np.uint32))
 
 
-@pytest.mark.skipif(not po.ref_available(), reason="oracle/_ref not built (needs /root/reference)")
 def test_port_delogo_and_calcfade2_equal_the_reference_code_live():
     """Round 2: AMTEraseLogo::Delogo and CalcFade2 (LogoScan.hpp:1248-1315) are compiled from the reference's own lines into
     oracle/_ref; the plain-C port (which the GPU erase kernel and the product's amtk_calc_fade2 are tested against) must
     reproduce them exactly: pixel bytes for Delogo (rounding, clamping, per-field pitches), the selected fades for
-    CalcFade2 incl. the double-offset quirk (:1273-1275) and the clip-end clamps."""
-    if not po.ref_has_erase():
-        pytest.skip("prebuilt oracle/_ref predates the Delogo/CalcFade2 extraction")
-    rng = np.random.default_rng(11)
-    for dtype, maxv in ((np.uint8, 255.0), (np.uint16, 1023.0)):
-        for (w, h, lp, ip) in ((64, 64, 64, 96), (32, 16, 64, 200), (7, 5, 7, 7)):       # field passes: logopitch 2w, imgpitch 2*pitch
-            img = rng.integers(0, int(maxv) + 1, size=(h, ip)).astype(dtype)
-            A = rng.uniform(0.8, 1.6, size=h * lp).astype(np.float32)
-            B = rng.uniform(-0.6, 0.1, size=h * lp).astype(np.float32)
-            for fade in (0.0, 0.1, 0.3, 0.5, 0.9, 1.0):
-                a, b = img.copy(), img.copy()
-                po.or_delogo(a, A, B, fade, maxv, logopitch=lp, imgpitch=ip, w=w, h=h)
+    CalcFade2 incl. the double-offset quirk (:1273-1275) and the clip-end clamps.  The reference's results are stored in
+    tests/golden/ref_cases.json and also computed live where oracle/_ref is built."""
+    live = po.ref_has_erase()
+    delogo, fade2 = ri.delogo_and_calc_fade2_cases()
+    want = iter(REF["delogo_sha"])
+    for dtype, maxv, w, h, lp, ip, img, A, B in delogo:
+        for fade in ri.DELOGO_FADES:
+            a = img.copy()
+            po.or_delogo(a, A, B, fade, maxv, logopitch=lp, imgpitch=ip, w=w, h=h)
+            assert digest(a) == next(want), (dtype, w, h, fade)
+            if live:
+                b = img.copy()
                 po.ref_delogo(b, A, B, fade, maxv, logopitch=lp, imgpitch=ip, w=w, h=h)
                 assert np.array_equal(a, b), (dtype, w, h, fade)
-                assert fade == 0.0 or not np.array_equal(a, img)
-    for N in (1, 5, 8, 9, 23, 64, 101):
-        rec = rng.uniform(0.0, 1.0, size=(N, 33)).astype(np.float32)
-        # sudden appear / disappear patterns so that both branches of :1295-1314 are taken
-        for k in range(N):
-            rec[k, : 11] += np.abs(np.arange(11) - (0 if (k // 7) % 2 == 0 else 10)) * np.float32(0.5)
+            assert fade == 0.0 or not np.array_equal(a, img)
+    for N, rec in fade2:
+        want_n = np.array(REF["calc_fade2_bits"][str(N)], np.uint32).view(np.float32).reshape(N, 2)
         took = set()
         for n in range(N):
-            want = po.ref_calc_fade2(rec, N, n)
             got = po.or_calc_fade2(rec, N, n)
-            assert got == want, (N, n, got, want)
-            took.add(want[0] == want[1])
+            assert bits(got) == bits(want_n[n]), (N, n, got, want_n[n])
+            if live:
+                assert po.ref_calc_fade2(rec, N, n) == got, (N, n)
+            took.add(bool(want_n[n, 0] == want_n[n, 1]))
         if N >= 23:
             assert took == {True, False}
 
 
-@pytest.mark.skipif(not po.ref_available(), reason="oracle/_ref not built (needs /root/reference)")
 def test_reference_mergefield_is_the_even_odd_row_weave_live():
     """AMTSource::MergeField / Copy1 / Copy2 compiled from the reference's own lines (AMTSource.hpp:291-355): even rows of
     every plane from `top`, odd rows from `bottom`, NV12 chroma de-interleaved -- the statement the GPU weave kernel
-    (amtk_weave_frames) is tested against on the device."""
-    if not po.ref_has_mergefield():
-        pytest.skip("prebuilt oracle/_ref predates the MergeField extraction")
-    rng = np.random.default_rng(5)
-    for (w, h) in ((16, 8), (208, 72), (64, 36)):      # heights are multiples of 4: Copy1 writes row pairs of the chroma planes too
+    (amtk_weave_frames) is tested against on the device.  The reference's outputs are stored as digests in
+    tests/golden/ref_cases.json and also computed live where oracle/_ref is built."""
+    live = po.ref_has_mergefield()
+    for k, (w, h, t, b) in enumerate(ri.mergefield_cases()):
         ysz, cw, ch = w * h, w // 2, h // 2
-        t = rng.integers(0, 256, ysz + 2 * cw * ch).astype(np.uint8)
-        b = rng.integers(0, 256, ysz + 2 * cw * ch).astype(np.uint8)
-        got = po.ref_merge_field(t, b, w, h)
+        exp = t.copy()
         for (o, rows, cols) in ((0, h, w), (ysz, ch, cw), (ysz + cw * ch, ch, cw)):
-            exp = t[o:o + rows * cols].reshape(rows, cols).copy()
-            exp[1::2] = b[o:o + rows * cols].reshape(rows, cols)[1::2]
-            assert np.array_equal(got[o:o + rows * cols].reshape(rows, cols), exp)
+            exp[o:o + rows * cols].reshape(rows, cols)[1::2] = b[o:o + rows * cols].reshape(rows, cols)[1::2]
+        g = REF["mergefield"][k]
+        assert (g["w"], g["h"]) == (w, h)
+        assert digest(exp) == g["planar_sha"] and digest(exp) == g["nv12_sha"], (w, h)
+        if live:
+            assert np.array_equal(po.ref_merge_field(t, b, w, h), exp)
+            assert np.array_equal(po.ref_merge_field(ri.to_nv12(t, w, h), ri.to_nv12(b, w, h), w, h, nv12=True), exp)
 
-        def to_nv12(a):
-            uv = np.stack([a[ysz:ysz + cw * ch], a[ysz + cw * ch:]], axis=1).reshape(-1)
-            return np.concatenate([a[:ysz], uv])
-        assert np.array_equal(po.ref_merge_field(to_nv12(t), to_nv12(b), w, h, nv12=True), got)
 
-
-@pytest.mark.skipif(not po.ref_available(), reason="oracle/_ref not built (needs /root/reference)")
 def test_reference_frame_drivers_equal_their_restated_compositions_live():
     """AMTAnalyzeLogo::GetFrameT (LogoScan.hpp:1119-1161) and LogoFrame::ScanFrame (:1543-1568) compiled from the reference's
-    own lines: the compositions the parity tests use (ref_analyze_frame / ref_scan_frame: the reference's DeintY, CopyY and
+    own lines (results stored in tests/golden/ref_cases.json): the compositions the parity tests use (DeintY, CopyY and
     EvaluateLogo called in the order those functions call them) give the same bits, including the source-frame clamp at the
-    clip end (:1133), the |.| of every evaluation, and the (0, -1) result for invalid or wrong-sized logos (:1551-1558)."""
-    if not po.ref_has_drivers():
-        pytest.skip("prebuilt oracle/_ref predates the GetFrameT/ScanFrame extraction")
-    w, h, imgx, imgy, N = 256, 128, 160, 32, 13
-    lg = synth.make_logo(64, 64)
-    fr = synth.make_frames(40, N, w, h, device="cpu", logo=lg, imgx=imgx, imgy=imgy, logo_period=12).numpy()
-    raw = po.RefLogo.create(lg["data"], 64, 64, w, h, imgx, imgy)
+    clip end (:1133), the |.| of every evaluation, and the (0, -1) result for invalid or wrong-sized logos (:1551-1558).
+    Checked for the port's compositions (or_analyze_frame / scan_frame) always, and where oracle/_ref is built for the
+    reference's (ref_analyze_frame / ref_scan_frame, the oracle of tests/test_gpu_parity_sizes.py there) against the live
+    drivers."""
+    w, h, imgx, imgy, lg, fr = ri.drivers_clip()
+    N = fr.shape[0]
+    raw = po.OracleLogo.create(lg["data"], 64, 64, w, h, imgx, imgy)
     de, top, bot = raw.deint().create_mask(0.35), raw.field(0).create_mask(0.35), raw.field(1).create_mask(0.35)
     Y = fr[:, : w * h].reshape(N, h, w)
+    g = REF["drivers"]
     for n in range((N + 7) // 8):
-        got = po.ref_analyze_getframe(de, top, bot, fr, w, h, n)
-        want = np.stack([po.ref_analyze_frame(de, top, bot, Y[min(N - 1, 8 * n + i)]) for i in range(8)])
-        assert np.array_equal(got.view(np.uint32), want.view(np.uint32)), n
-    other = po.RefLogo.create(lg["data"], 64, 64, w + 16, h, imgx, imgy).deint().create_mask(0.35)      # made for another frame size
-    for k in (0, 5, N - 1):
-        got = po.ref_scan_frame_code([de, None, other], fr[k], w, h)
-        assert np.array_equal(got[0].view(np.uint32), po.ref_scan_frame(de, Y[k]).view(np.uint32))
+        want = np.stack([po.or_analyze_frame(de, top, bot, Y[min(N - 1, 8 * n + i)]) for i in range(8)])
+        assert bits(want) == g["getframe_bits"][n], n
+    assert g["scanframe_frames"] == list(ri.DRIVER_SCAN_FRAMES)
+    for k, i in enumerate(ri.DRIVER_SCAN_FRAMES):
+        got = np.array(g["scanframe_bits"][k], np.uint32).view(np.float32).reshape(3, 2)
+        assert bits(got[0]) == bits(de.scan_frame(Y[i]))
         assert tuple(got[1]) == (0.0, -1.0) and tuple(got[2]) == (0.0, -1.0)
+    if po.ref_has_drivers():
+        rraw = po.RefLogo.create(lg["data"], 64, 64, w, h, imgx, imgy)
+        rde, rtop, rbot = rraw.deint().create_mask(0.35), rraw.field(0).create_mask(0.35), rraw.field(1).create_mask(0.35)
+        for n in range((N + 7) // 8):
+            got = po.ref_analyze_getframe(rde, rtop, rbot, fr, w, h, n)
+            want = np.stack([po.ref_analyze_frame(rde, rtop, rbot, Y[min(N - 1, 8 * n + i)]) for i in range(8)])
+            assert np.array_equal(got.view(np.uint32), want.view(np.uint32)), n
+            assert bits(got) == g["getframe_bits"][n], n
+        other = po.RefLogo.create(lg["data"], 64, 64, w + 16, h, imgx, imgy).deint().create_mask(0.35)      # made for another frame size
+        for k, i in enumerate(ri.DRIVER_SCAN_FRAMES):
+            got = po.ref_scan_frame_code([rde, None, other], fr[i], w, h)
+            assert np.array_equal(got[0].view(np.uint32), po.ref_scan_frame(rde, Y[i]).view(np.uint32))
+            assert tuple(got[1]) == (0.0, -1.0) and tuple(got[2]) == (0.0, -1.0)
+            assert bits(got) == g["scanframe_bits"][k]
 
 
 def test_erase_and_weave_golden_from_the_reference_code(tmp_path):
